@@ -2,7 +2,7 @@
 """bench.py — residuals/sec per Levenberg-Marquardt iteration of the continuous-time IMU-camera calibration solve.
 
 Contract (see DESIGN.md "Measurement"):
-  python bench.py --gpus N --steps K --warmup W [--impl reference] [--config 4]
+  python bench.py --gpus N --steps K --warmup W [--impl reference] [--config 4] [--dump-outputs DIR]
   * workload  = BASELINE.json configs[3]: ExtendedUnified, 3000 frames x 144 corners, 1 kHz IMU (the config the metric's
                 target is quoted on; fits one B200).  N > 1 shards the residuals by time slice, NCCL all-reduce of the
                 packed J^T J / J^T r buffer (strong scaling).
@@ -36,6 +36,21 @@ from openimucameracalibrator_b200 import synthetic as syn  # noqa: E402
 FLAGS = capi.FLAG_SPLINE | capi.FLAG_T_I_C      # the hot CLI's stage-1 flags with a known gravity axis (app :200-215)
 METRIC = "residuals/sec per LM iter"
 UNIT = "residuals/s"
+# summary fields that depend only on the computation (timings and launch counts are left out)
+DUMP_SUMMARY_FIELDS = ("iterations", "successful_steps", "termination", "num_residuals", "num_tangent", "initial_cost", "final_cost", "mean_reproj_error")
+
+
+def dump_outputs(out_dir, api, summ, prefix=""):
+    """--dump-outputs: what one LM-iteration step hands its caller, as float64 DIR/<prefix><name>.npy -- the updated spline knots,
+    T_i_c and line delay read back from the handle, and the returned summary.  Every step starts from the same state and the
+    inputs are seeded, so two builds run with the same arguments can be compared file for file."""
+    os.makedirs(out_dir, exist_ok=True)
+    so3, r3, ba, bg = api.get_knots()
+    arrays = {"so3_knots": so3, "r3_knots": r3, "accel_bias_knots": ba, "gyro_bias_knots": bg, "T_i_c": api.get_T_i_c(),
+              "line_delay": [api.get_line_delay()]}
+    arrays.update({"summary_" + k: [getattr(summ, k)] for k in DUMP_SUMMARY_FIELDS})
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def workload_name(cfg):
@@ -154,9 +169,11 @@ def run_reference(args, cfg):
     times = []
     for i in range(args.warmup + args.steps):
         o.set_knots(so3, r3, ba, bg); o.set_T_i_c(T0); o.set_line_delay(ld0)
-        t = time.perf_counter(); o.lm_iterations(1, FLAGS); dt = time.perf_counter() - t
+        t = time.perf_counter(); summ = o.lm_iterations(1, FLAGS); dt = time.perf_counter() - t
         if i >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, o, summ)
     ms = 1e3 * float(np.mean(times))
     value = nres / (ms * 1e-3)
     full = c.n_frames == cfg.n_frames
@@ -206,14 +223,15 @@ def run_batch_of_eight(args):
         if sampler: sampler.sample()                # under load (the fill is running), outside the wall-clock bracket of any round
         sync()
         t0 = time.perf_counter()
-        n_l = 0
-        for a in handles:
-            n_l += a.lm_iterations(1, FLAGS).gpu_launches     # each call ends with a stream synchronisation
+        summs = [a.lm_iterations(1, FLAGS) for a in handles]     # each call ends with a stream synchronisation
         torch.cuda.synchronize()
         if i >= args.warmup:
-            total_ms += 1e3 * (time.perf_counter() - t0); launches += n_l
+            total_ms += 1e3 * (time.perf_counter() - t0); launches += sum(s.gpu_launches for s in summs)
     sync()
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs:
+        for k, a, s in zip(mine, handles, summs):
+            dump_outputs(args.dump_outputs, a, s, prefix=f"seq{k}_")
     tot_res = nres
     if world > 1:
         t = torch.tensor([total_ms, float(nres)], dtype=torch.float64, device=f"cuda:{local}")
@@ -241,6 +259,7 @@ def main():
     ap.add_argument("--cpu-baseline-steps", type=int, default=3)
     ap.add_argument("--e2e-steps", type=int, default=3)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed as DIR/<name>.npy (float64)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.config == 5:
@@ -324,6 +343,8 @@ def main():
     barrier()
     clocks = sampler.stop() if sampler else None
     gc.enable()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, api, summ)
     total_ms = float(np.sum(step_ms))
     if world > 1:
         t = torch.tensor([total_ms], dtype=torch.float64, device=f"cuda:{local}"); dist.all_reduce(t, op=dist.ReduceOp.MAX); total_ms = float(t.item())
@@ -412,7 +433,7 @@ def main():
     cpu = None
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         import copy
-        ns = copy.copy(args); ns.steps = args.cpu_baseline_steps; ns.warmup = 0
+        ns = copy.copy(args); ns.steps = args.cpu_baseline_steps; ns.warmup = 0; ns.dump_outputs = None
         ref = run_reference(ns, cfg)
         cpu = ref["cpu_baseline"]
 

@@ -1,6 +1,7 @@
 """Ad-hoc GPU vs oracle comparison (developer tool; the real parity tests live in test_*.py)."""
-import sys, time, numpy as np
-sys.path.insert(0, '/root/repo'); sys.path.insert(0, '/root/repo/tests')
+import os, sys, time, numpy as np
+HERE = os.path.dirname(os.path.abspath(__file__))
+sys.path.insert(0, os.path.dirname(HERE)); sys.path.insert(0, HERE)
 from oracle_api import new_oracle
 from openimucameracalibrator_b200 import synthetic as syn, _capi as capi, calibrator
 from openimucameracalibrator_b200 import camera_models as cm
