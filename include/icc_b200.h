@@ -208,6 +208,19 @@ icc_status icc_evaluate(icc_handle* h, int flags, double* cost, double* residual
 /* J^T J V for nvec caller vectors (canonical tangent order, one vector after the other) from the packed normal equations of the
  * current state: full-size parity of the reduced system without a dense Hessian (evaluation helper, like icc_evaluate). */
 icc_status icc_normal_matvec(icc_handle* h, int flags, int nvec, const double* V, double* HV);
+/* The elimination plan of the damped solve under `flags` (works on a host-only handle): plan[0..12] = valid, P (level-0 chunks),
+ * w (separator width), len, rem (chunk c owns len + (c < rem) interior knot columns), L (cyclic-reduction levels), kd (half
+ * bandwidth), nb (border columns), nk (knot columns), WS_A (level-0 window slots), cl_global, cs_global (dense border blocks in
+ * global memory), stage0 (level-0 back-substitution staged in shared memory); plan[13..15] reserved (0).  chunks = 0: the
+ * library's own choice; chunks > 0 forces the level-0 chunk count, then clamped and halved like the automatic choice. */
+icc_status icc_get_solver_plan(icc_handle* h, int flags, int chunks, int32_t* plan16);
+/* One damped solve at the current state (test surface): one Jacobian evaluation, its Jacobi scale S (options.jacobi_scaling),
+ * D = clamp(diag(S H S), min_lm_diagonal, max_lm_diagonal) / radius, (S H S + D) y = -S g on the plan of `chunks` (as in
+ * icc_get_solver_plan).  Outputs in canonical tangent order, each nullable: cost, gradient g and hessian_dense H (n x n, small
+ * problems only) of the evaluation the solve consumed, scale S, lm_diag D, delta = S y, model_change = 1/2 (y^T D y - y^T S g).
+ * The state and the LM bookkeeping are not changed.  ICC_ERR_UNSUPPORTED: no valid plan; ICC_ERR_NUMERIC: a pivot broke down. */
+icc_status icc_solve_step(icc_handle* h, int flags, double radius, int chunks, double* cost, double* gradient, double* hessian_dense,
+                          double* scale, double* lm_diag, double* delta, double* model_change);
 icc_status icc_lm_iterations(icc_handle* h, int n, int flags, icc_summary* summary);
 /* Run `n` bare residual+Jacobian+normal-equation evaluations (the residual-eval kernels only); device ms per evaluation. */
 icc_status icc_time_evaluations(icc_handle* h, int n, int flags, int with_jacobian, double* ms_per_eval);

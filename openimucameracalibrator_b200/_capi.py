@@ -21,6 +21,8 @@ FLAG_CAM_INTRINSICS, FLAG_TIME_OFFSET = 512, 1024     # north-star extensions (t
 STATUS_NAMES = {0: "ICC_OK", 1: "ICC_ERR_INVALID_ARGUMENT", 2: "ICC_ERR_NO_DEVICE", 3: "ICC_ERR_CUDA", 4: "ICC_ERR_STATE",
                 5: "ICC_ERR_UNSUPPORTED", 6: "ICC_ERR_NUMERIC"}
 TERMINATION = {0: "max_iterations", 1: "function_tolerance", 2: "parameter_tolerance", 3: "gradient_tolerance", 4: "failure"}
+# icc_get_solver_plan's int32[16] (the last three are reserved)
+PLAN_FIELDS = ("valid", "P", "w", "len", "rem", "L", "kd", "nb", "nk", "WS_A", "cl_global", "cs_global", "stage0")
 
 
 class InitParams(C.Structure):
@@ -378,6 +380,23 @@ class CApi:
         H = np.zeros((n, n)) if hessian else None
         self._call("evaluate", [C.c_int, c_double_p, c_double_p, c_double_p, c_double_p], int(flags), C.byref(cost), _dp(r), _dp(g), _dp(H))
         return cost.value, r, g, H
+
+    def solver_plan(self, flags, chunks=0) -> dict:
+        """Elimination plan of the damped solve (icc_get_solver_plan); chunks > 0 forces the level-0 chunk count."""
+        p = np.zeros(16, dtype=np.int32)
+        self._call("get_solver_plan", [C.c_int, C.c_int, c_int32_p], int(flags), int(chunks), p.ctypes.data_as(c_int32_p))
+        return dict(zip(PLAN_FIELDS, (int(v) for v in p)))
+
+    def solve_step(self, flags, radius, chunks=0, hessian=True) -> dict:
+        """One damped solve at the current state (icc_solve_step): cost, gradient, hessian (None unless asked), scale, lm_diag,
+        delta, model_change, all from the one evaluation the solve consumed, canonical tangent order."""
+        n = self.num_tangent(flags)
+        cost, mc = C.c_double(), C.c_double()
+        g, s, d, x = np.zeros(n), np.zeros(n), np.zeros(n), np.zeros(n)
+        H = np.zeros((n, n)) if hessian else None
+        self._call("solve_step", [C.c_int, C.c_double, C.c_int] + [c_double_p] * 7, int(flags), float(radius), int(chunks),
+                   C.byref(cost), _dp(g), _dp(H), _dp(s), _dp(d), _dp(x), C.byref(mc))
+        return dict(cost=cost.value, gradient=g, hessian=H, scale=s, lm_diag=d, delta=x, model_change=mc.value)
 
 
 def _normal_matvec(self, flags, V):

@@ -491,6 +491,19 @@ icc_status mean_reproj(icc_handle* h, double* out) {
   return ICC_OK;
 }
 
+// Dense J^T J (canonical tangent order, row-major) from the packed banded + bordered normal equations read back to the host.
+void dense_hessian(const icc_handle* h, const std::vector<double>& ne, double* out) {
+  const DeviceProblem& P = h->P;
+  const int n = h->n_tan;
+  auto get = [&](int a, int b) -> double {
+    const int lo = std::min(a, b), hi = std::max(a, b);
+    if (hi < P.nk) return hi - lo <= P.kd ? ne[(size_t)lo * P.ldb + (hi - lo)] : 0.0;
+    if (lo < P.nk) return ne[P.ne_off_E + (size_t)lo * P.nb + (hi - P.nk)];
+    return ne[P.ne_off_C + (size_t)(hi - P.nk) * P.nb + (lo - P.nk)];
+  };
+  for (int i = 0; i < n; ++i) for (int j = 0; j < n; ++j) out[(size_t)i * n + j] = get(h->perm[i], h->perm[j]);
+}
+
 // Levenberg-Marquardt with Ceres TrustRegionMinimizer semantics (options: impl.h:254-266 + Ceres 2.1 defaults).
 icc_status run_lm(icc_handle* h, int max_iters, int flags, bool check_convergence, icc_summary* out) {
   using clk = std::chrono::steady_clock;
@@ -1346,15 +1359,7 @@ icc_status icc_evaluate(icc_handle* h, int flags, double* cost, double* residual
   CU(cudaStreamSynchronize(h->stream));
   if (cost) *cost = ne[P.ne_off_cost];
   if (gradient) for (int i = 0; i < n; ++i) gradient[i] = ne[P.ne_off_g + h->perm[i]];
-  if (hessian) {
-    auto get = [&](int a, int b) -> double {
-      const int lo = std::min(a, b), hi = std::max(a, b);
-      if (hi < P.nk) return hi - lo <= P.kd ? ne[(size_t)lo * P.ldb + (hi - lo)] : 0.0;
-      if (lo < P.nk) return ne[P.ne_off_E + (size_t)lo * P.nb + (hi - P.nk)];
-      return ne[P.ne_off_C + (size_t)(hi - P.nk) * P.nb + (lo - P.nk)];
-    };
-    for (int i = 0; i < n; ++i) for (int j = 0; j < n; ++j) hessian[(size_t)i * n + j] = get(h->perm[i], h->perm[j]);
-  }
+  if (hessian) dense_hessian(h, ne, hessian);
   return ICC_OK;
 }
 
@@ -1390,6 +1395,64 @@ icc_status icc_normal_matvec(icc_handle* h, int flags, int nvec, const double* V
     }
     for (int i = 0; i < n; ++i) HV[(size_t)v * n + i] = y[h->perm[i]];
   }
+  return ICC_OK;
+}
+
+// The elimination plan of the damped solve for `flags` (host only: works on a host-only handle).  chunks > 0 forces the level-0
+// chunk count, which then goes through the same clamping and halving as the automatic choice.
+icc_status icc_get_solver_plan(icc_handle* h, int flags, int chunks, int32_t* plan16) {
+  if (!h || !plan16 || chunks < 0) return ICC_ERR_INVALID_ARGUMENT;
+  if (!h->initialised) return fail(h, ICC_ERR_STATE, "icc_batch_init_spline must be called first");
+  icc_status s = configure(h, flags); if (s != ICC_OK) return s;
+  solve_plan_info(h->P, chunks, plan16);
+  return ICC_OK;
+}
+
+// One damped solve at the current state, outside the LM driver: one Jacobian evaluation, the Jacobi scale of THAT evaluation, one
+// launch_solve.  Outputs (canonical tangent order, each nullable) all come from the same evaluation, so a host reference can rebuild
+// exactly the system the kernels factored.  Leaves the state, the LM scale and the LM bookkeeping untouched.
+icc_status icc_solve_step(icc_handle* h, int flags, double radius, int chunks, double* cost, double* gradient, double* hessian_dense,
+                          double* scale, double* lm_diag, double* delta, double* model_change) {
+  if (!h || !(radius > 0.0) || chunks < 0) return ICC_ERR_INVALID_ARGUMENT;
+  NEED_DEVICE();
+  if (!h->initialised) return fail(h, ICC_ERR_STATE, "icc_batch_init_spline must be called first");
+  CU(cudaSetDevice(h->device));
+  icc_status s = configure(h, flags); if (s != ICC_OK) return s;
+  const DeviceProblem& P = h->P;
+  const int n = h->n_tan;
+  if (n == 0) return fail(h, ICC_ERR_INVALID_ARGUMENT, "no free parameters for these flags");
+  int32_t plan[16]; solve_plan_info(P, chunks, plan);
+  if (!plan[0]) return fail(h, ICC_ERR_UNSUPPORTED, "the border (bias knots + globals) is too wide for the solver's shared-memory plans");
+  DevBuf<double> d_scale, d_delta, d_scal, d_ws;
+  CU(d_scale.alloc((size_t)n)); CU(d_delta.alloc((size_t)n)); CU(d_scal.alloc(SC_COUNT));
+  double* ws = h->d_ws.p;
+  if (chunks > 0) { CU(d_ws.alloc(solve_workspace_doubles(P, chunks))); ws = d_ws.p; }
+  s = eval_jacobian(h, h->st[h->cur].view(), nullptr); if (s != ICC_OK) { cudaStreamSynchronize(h->stream); return s; }
+  CU(cudaMemsetAsync(d_scal.p, 0, SC_COUNT * sizeof(double), h->stream));
+  launch_compute_scale(P, d_scale.p, h->opt.jacobi_scaling, d_scal.p, h->stream);
+  SolveParams sp; sp.radius = radius; sp.min_diag = h->opt.min_lm_diagonal; sp.max_diag = h->opt.max_lm_diagonal; sp.jacobi_scaling = h->opt.jacobi_scaling;
+  const int se = launch_solve(P, d_scale.p, sp, ws, d_delta.p, d_scal.p, h->stream, chunks);
+  if (se) { cudaStreamSynchronize(h->stream); return fail(h, ICC_ERR_CUDA, std::string("solver launch: ") + cudaGetErrorString(cudaGetLastError())); }
+  std::vector<double> ne((size_t)P.ne_size), sc_h((size_t)n), dl_h((size_t)n);
+  double sc[SC_COUNT];
+  CU(cudaMemcpyAsync(ne.data(), P.ne, ne.size() * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaMemcpyAsync(sc_h.data(), d_scale.p, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaMemcpyAsync(dl_h.data(), d_delta.p, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaMemcpyAsync(sc, d_scal.p, sizeof sc, cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaStreamSynchronize(h->stream));
+  if (sc[SC_OK] != 1.0) return fail(h, ICC_ERR_NUMERIC, "the factorisation met a non-positive pivot");
+  // diagonal of H in solver order; the LM diagonal is the same expression as the kernels' lm_d2
+  auto diag = [&](int i) { return i < P.nk ? ne[(size_t)i * P.ldb] : ne[P.ne_off_C + (size_t)(i - P.nk) * P.nb + (i - P.nk)]; };
+  for (int i = 0; i < n; ++i) {
+    const int j = h->perm[i];
+    if (gradient) gradient[i] = ne[P.ne_off_g + j];
+    if (scale) scale[i] = sc_h[j];
+    if (lm_diag) lm_diag[i] = std::fmin(std::fmax(diag(j) * sc_h[j] * sc_h[j], sp.min_diag), sp.max_diag) / sp.radius;
+    if (delta) delta[i] = dl_h[j];
+  }
+  if (cost) *cost = ne[P.ne_off_cost];
+  if (model_change) *model_change = sc[SC_MODEL_CHANGE];
+  if (hessian_dense) dense_hessian(h, ne, hessian_dense);
   return ICC_OK;
 }
 

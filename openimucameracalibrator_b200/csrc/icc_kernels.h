@@ -99,8 +99,11 @@ int launch_eval(const DeviceProblem& P, const DeviceState& S, bool with_jacobian
 void launch_compute_scale(const DeviceProblem& P, double* scale, int jacobi, double* scal, cudaStream_t st);
 // banded + bordered Cholesky solve of (S H S + D) y = -S g ; delta = S y (solver order) ; model cost change
 // returns 0, 1 = no elimination plan fits the shared-memory limits (border far too wide), 2 = a launch failed
-int launch_solve(const DeviceProblem& P, const double* scale, SolveParams sp, double* workspace, double* delta, double* scal, cudaStream_t st);
-size_t solve_workspace_doubles(const DeviceProblem& P);
+// forced_chunks > 0 replaces the plan's own level-0 chunk count (then clamped and halved exactly like the automatic choice)
+int launch_solve(const DeviceProblem& P, const double* scale, SolveParams sp, double* workspace, double* delta, double* scal, cudaStream_t st, int forced_chunks = 0);
+size_t solve_workspace_doubles(const DeviceProblem& P, int forced_chunks = 0);
+// the elimination plan launch_solve would run: valid, P, w, len, rem, L, kd, nb, nk, WS_A, cl_global, cs_global, stage0, 0, 0, 0
+void solve_plan_info(const DeviceProblem& P, int forced_chunks, int32_t plan[16]);
 // candidate = Plus(current, delta) ; step / x squared norms
 void launch_update(const DeviceProblem& P, const DeviceState& cur, const DeviceState& cand, const double* delta, double max_ba, double max_bg, double* scal, cudaStream_t st);
 // knot initialisation from the per-view pose priors (icc_init.cu): q_wc / p_wc / t_vis in view-time order, T_c_i = T_i_c^-1 (x,y,z,w,tx,ty,tz)

@@ -978,12 +978,15 @@ size_t smem_CR(const DeviceProblem& P, const SolvePlan& pl) {
 
 // Chunking of the knot columns: leaves cost their interior length in sequential column eliminations, every cyclic-reduction
 // level a dense w = kd column front plus two launches.
-// Wide borders (bias splines active) keep P = 1: the left-separator coupling would not fit the shared-memory window.
+// Wide borders keep chunking: the dense border blocks move to HBM (cl_global / cs_global) and the chunk count halves only
+// when a kernel's shared memory still exceeds the limit.
+// forced > 0 replaces the chunk count of the cost model and of ICC_SOLVER_CHUNKS / ICC_SOLVER_LEAF (tests pin every plan with it).
 int env_int(const char* name, int dflt) { const char* v = getenv(name); return v && *v ? atoi(v) : dflt; }
-SolvePlan make_plan(const DeviceProblem& P) {
+SolvePlan make_plan(const DeviceProblem& P, int forced) {
   SolvePlan pl; memset(&pl, 0, sizeof pl);
   const int nk = P.nk, kd = P.kd, nb = P.nb;
-  static const int forced_chunks = env_int("ICC_SOLVER_CHUNKS", 0), leaf_cols = env_int("ICC_SOLVER_LEAF", 0);
+  static const int env_chunks = env_int("ICC_SOLVER_CHUNKS", 0), leaf_cols = env_int("ICC_SOLVER_LEAF", 0);
+  const int forced_chunks = forced > 0 ? forced : env_chunks;
   int Pn = 1;
   if (nk > 0 && kd > 0) {
     // P = 2^k chunks give a complete elimination tree of k-1 reduction levels; measured on B200: ~0.45 us per leaf column
@@ -1035,10 +1038,16 @@ SolvePlan make_plan(const DeviceProblem& P) {
 
 }  // namespace
 
-size_t solve_workspace_doubles(const DeviceProblem& P) {
-  const SolvePlan pl = make_plan(P);
+size_t solve_workspace_doubles(const DeviceProblem& P, int forced_chunks) {
+  const SolvePlan pl = make_plan(P, forced_chunks);
   if (!pl.valid) return 16;
   return carve(nullptr, P.nk, P.nb, P.ldb, pl).total;
+}
+
+void solve_plan_info(const DeviceProblem& P, int forced_chunks, int32_t plan[16]) {
+  const SolvePlan pl = make_plan(P, forced_chunks);
+  const int32_t v[16] = {pl.valid, pl.P, pl.w, pl.len, pl.rem, pl.L, P.kd, P.nb, P.nk, pl.WS_A, pl.cl_global, pl.cs_global, pl.stage0, 0, 0, 0};
+  memcpy(plan, v, sizeof v);
 }
 
 void launch_compute_scale(const DeviceProblem& P, double* scale, int jacobi, double* scal, cudaStream_t st) {
@@ -1048,8 +1057,8 @@ void launch_compute_scale(const DeviceProblem& P, double* scale, int jacobi, dou
   count_launch();
 }
 
-int launch_solve(const DeviceProblem& P, const double* scale, SolveParams sp, double* workspace, double* delta, double* scal, cudaStream_t st) {
-  const SolvePlan pl = make_plan(P);
+int launch_solve(const DeviceProblem& P, const double* scale, SolveParams sp, double* workspace, double* delta, double* scal, cudaStream_t st, int forced_chunks) {
+  const SolvePlan pl = make_plan(P, forced_chunks);
   if (!pl.valid) return 1;                       // border too wide / problem too small for any plan within the shared-memory limit
   const SolveWs ws = carve(workspace, P.nk, P.nb, P.ldb, pl);
   static size_t cfgA = 0, cfgR = 0, cfgB = 0, cfgC = 0, cfgCR = 0;

@@ -893,6 +893,39 @@ void inner_iterations(Oracle& o) {
 // -------------------------------------------------------------------------------------------------------------
 struct LMResult { icc_summary sum; };
 
+// Jacobi column scaling (solver order): S_ii = 1 / (1 + sqrt(H_ii)), or the identity without it.
+std::vector<double> jacobi_scale(const Normal& ne, bool jacobi) {
+  const int n = ne.nk + ne.nb;
+  std::vector<double> scale(n, 1.0);
+  if (jacobi) for (int i = 0; i < n; ++i) scale[i] = 1.0 / (1.0 + std::sqrt(i < ne.nk ? ne.band[size_t(i) * (ne.kd + 1)] : ne.C[size_t(i - ne.nk) * ne.nb + (i - ne.nk)]));
+  return scale;
+}
+
+// One LevenbergMarquardtStrategy::ComputeStep (solver order): scaled system Hs = S H S, gs = S g; the clamped diagonal
+// diag = clamp(diag(Hs), min_lm_diagonal, max_lm_diagonal) (kept from the previous call when reuse_diagonal); D2 = diag / radius;
+// (Hs + D2) y = -gs; model_change = -y^T gs - 1/2 y^T Hs y.  Returns false on a Cholesky breakdown.
+struct LmStep { Normal sc; std::vector<double> diag, D2, rhs, y; double model_change = 0; };
+bool lm_step(const Normal& ne, const std::vector<double>& scale, double radius, const icc_solver_options& opt, bool reuse_diagonal, LmStep& st) {
+  const int n = ne.nk + ne.nb;
+  Normal& sc = st.sc;
+  sc = ne;
+  for (int j = 0; j < ne.nk; ++j) { const int m = std::min(ne.kd, ne.nk - 1 - j); for (int i = 0; i <= m; ++i) sc.band[size_t(j) * (ne.kd + 1) + i] *= scale[j] * scale[j + i]; }
+  for (int b = 0; b < ne.nb; ++b) for (int j = 0; j < ne.nk; ++j) sc.E[size_t(b) * ne.nk + j] *= scale[ne.nk + b] * scale[j];
+  for (int b = 0; b < ne.nb; ++b) for (int c = 0; c < ne.nb; ++c) sc.C[size_t(b) * ne.nb + c] *= scale[ne.nk + b] * scale[ne.nk + c];
+  st.rhs.resize(n); st.D2.resize(n); st.diag.resize(n, 0.0);
+  for (int i = 0; i < n; ++i) st.rhs[i] = -scale[i] * ne.g[i];
+  if (!reuse_diagonal) for (int i = 0; i < n; ++i) { const double dv = i < sc.nk ? sc.band[size_t(i) * (sc.kd + 1)] : sc.C[size_t(i - sc.nk) * sc.nb + (i - sc.nk)]; st.diag[i] = std::min(std::max(dv, opt.min_lm_diagonal), opt.max_lm_diagonal); }
+  for (int i = 0; i < n; ++i) st.D2[i] = st.diag[i] / radius;
+  st.model_change = 0;
+  if (!arrowhead_solve(sc, st.D2, st.rhs, st.y)) return false;
+  double yg = 0, yHy = 0;
+  for (int i = 0; i < n; ++i) yg += st.y[i] * (-st.rhs[i]);
+  for (int j = 0; j < sc.nk; ++j) { const int m = std::min(sc.kd, sc.nk - 1 - j); yHy += sc.band[size_t(j) * (sc.kd + 1)] * st.y[j] * st.y[j]; for (int i = 1; i <= m; ++i) yHy += 2.0 * sc.band[size_t(j) * (sc.kd + 1) + i] * st.y[j] * st.y[j + i]; }
+  for (int b = 0; b < sc.nb; ++b) { for (int j = 0; j < sc.nk; ++j) yHy += 2.0 * sc.E[size_t(b) * sc.nk + j] * st.y[sc.nk + b] * st.y[j]; for (int c = 0; c < sc.nb; ++c) yHy += sc.C[size_t(b) * sc.nb + c] * st.y[sc.nk + b] * st.y[sc.nk + c]; }
+  st.model_change = -yg - 0.5 * yHy;
+  return true;
+}
+
 void lm_solve(Oracle& o, int max_iters, int flags, bool check_convergence, icc_summary& S) {
   using clk = std::chrono::steady_clock;
   const auto t_start = clk::now();
@@ -904,48 +937,30 @@ void lm_solve(Oracle& o, int max_iters, int flags, bool check_convergence, icc_s
   double x_cost = 0;
   auto eval_jac = [&]() { auto t0 = clk::now(); evaluate(o, &x_cost, nullptr, &ne, nullptr, nres); t_jac += std::chrono::duration<double>(clk::now() - t0).count(); ++S.jacobian_evaluations; };
   std::vector<double> scale;   // solver order
-  auto diagH = [&](int i) { return i < ne.nk ? ne.band[size_t(i) * (ne.kd + 1)] : ne.C[size_t(i - ne.nk) * ne.nb + (i - ne.nk)]; };
   double radius = o.opt.initial_trust_region_radius, decrease_factor = 2.0;
   bool reuse_diagonal = false, ne_valid = false, first = true;
-  std::vector<double> diag(n, 0.0), D2(n), rhs(n), y(n), delta_canon(n);
+  std::vector<double> delta_canon(n);
   int invalid = 0;
   bool inner_enabled = o.inner_iterations;
   o.inner_iteration_steps = 0;
   S.termination = 0;
   auto grad_max = [&]() { double m = 0; for (double v : ne.g) m = std::max(m, std::fabs(v)); return m; };
-  Normal sc;
+  LmStep st;
   for (int it = 0; it < max_iters; ++it) {
     // Jacobian rebuilt lazily at the top of the iteration that needs it (same schedule as the CUDA driver)
     if (!ne_valid) {
       eval_jac(); ne_valid = true;
       if (first) {
         first = false; S.initial_cost = x_cost;
-        scale.assign(n, 1.0);
-        if (o.opt.jacobi_scaling) for (int i = 0; i < n; ++i) scale[i] = 1.0 / (1.0 + std::sqrt(diagH(i)));
+        scale = jacobi_scale(ne, o.opt.jacobi_scaling);
       }
       if (check_convergence && grad_max() <= o.opt.gradient_tolerance) { S.termination = 3; break; }
     }
     ++S.iterations;
-    // scaled system  Hs = S H S, gs = S g
-    sc = ne;
-    for (int j = 0; j < ne.nk; ++j) { const int m = std::min(ne.kd, ne.nk - 1 - j); for (int i = 0; i <= m; ++i) sc.band[size_t(j) * (ne.kd + 1) + i] *= scale[j] * scale[j + i]; }
-    for (int b = 0; b < ne.nb; ++b) for (int j = 0; j < ne.nk; ++j) sc.E[size_t(b) * ne.nk + j] *= scale[ne.nk + b] * scale[j];
-    for (int b = 0; b < ne.nb; ++b) for (int c = 0; c < ne.nb; ++c) sc.C[size_t(b) * ne.nb + c] *= scale[ne.nk + b] * scale[ne.nk + c];
-    for (int i = 0; i < n; ++i) rhs[i] = -scale[i] * ne.g[i];
-    if (!reuse_diagonal) for (int i = 0; i < n; ++i) { const double dv = i < sc.nk ? sc.band[size_t(i) * (sc.kd + 1)] : sc.C[size_t(i - sc.nk) * sc.nb + (i - sc.nk)]; diag[i] = std::min(std::max(dv, o.opt.min_lm_diagonal), o.opt.max_lm_diagonal); }
-    for (int i = 0; i < n; ++i) D2[i] = diag[i] / radius;
     auto t0 = clk::now();
-    const bool ok = arrowhead_solve(sc, D2, rhs, y);
+    const bool ok = lm_step(ne, scale, radius, o.opt, reuse_diagonal, st);
     t_lin += std::chrono::duration<double>(clk::now() - t0).count();
-    // model_cost_change = -y^T gs - 0.5 y^T Hs y
-    double model_change = 0;
-    if (ok) {
-      double yg = 0, yHy = 0;
-      for (int i = 0; i < n; ++i) yg += y[i] * (-rhs[i]);
-      for (int j = 0; j < sc.nk; ++j) { const int m = std::min(sc.kd, sc.nk - 1 - j); yHy += sc.band[size_t(j) * (sc.kd + 1)] * y[j] * y[j]; for (int i = 1; i <= m; ++i) yHy += 2.0 * sc.band[size_t(j) * (sc.kd + 1) + i] * y[j] * y[j + i]; }
-      for (int b = 0; b < sc.nb; ++b) { for (int j = 0; j < sc.nk; ++j) yHy += 2.0 * sc.E[size_t(b) * sc.nk + j] * y[sc.nk + b] * y[j]; for (int c = 0; c < sc.nb; ++c) yHy += sc.C[size_t(b) * sc.nb + c] * y[sc.nk + b] * y[sc.nk + c]; }
-      model_change = -yg - 0.5 * yHy;
-    }
+    double model_change = st.model_change;
     if (!ok || !(model_change > 0.0)) {
       if (++invalid >= o.opt.max_consecutive_invalid_steps) { S.termination = 4; break; }
       radius = radius / decrease_factor; decrease_factor *= 2.0; reuse_diagonal = true;
@@ -953,7 +968,7 @@ void lm_solve(Oracle& o, int max_iters, int flags, bool check_convergence, icc_s
       continue;
     }
     invalid = 0;
-    for (int c = 0; c < n; ++c) delta_canon[c] = y[o.perm[c]] * scale[o.perm[c]];
+    for (int c = 0; c < n; ++c) delta_canon[c] = st.y[o.perm[c]] * scale[o.perm[c]];
     State snap; save_state(o, snap);
     double step_sq, x_sq; apply_plus(o, delta_canon, step_sq, x_sq);
     double cand_cost; evaluate(o, &cand_cost, nullptr, nullptr, nullptr, nres); ++S.cost_evaluations;
@@ -1210,6 +1225,32 @@ icc_status icco_lm_iterations(void* h, int n, int flags, icc_summary* S) {
   if (!configure(o, flags)) return ICC_ERR_UNSUPPORTED;
   icc_summary s; lm_solve(o, n, flags, false, s);
   if (S) *S = s;
+  return ICC_OK;
+}
+// One damped solve at the current state, same contract as icc_solve_step (`chunks` has no meaning here: one sequential factorisation).
+icc_status icco_solve_step(void* h, int flags, double radius, int chunks, double* cost, double* gradient, double* hessian_dense,
+                           double* scale, double* lm_diag, double* delta, double* model_change) {
+  Oracle& o = *O(h);
+  if (!o.initialised) { o.err = "batch_init_spline first"; return ICC_ERR_STATE; }
+  if (!(radius > 0.0) || chunks < 0) return ICC_ERR_INVALID_ARGUMENT;
+  if (!configure(o, flags)) return ICC_ERR_UNSUPPORTED;
+  const int n = o.n_tan;
+  if (n == 0) return ICC_ERR_INVALID_ARGUMENT;
+  Normal ne; double c;
+  evaluate(o, &c, nullptr, &ne, nullptr, total_residuals(o));
+  const std::vector<double> s = jacobi_scale(ne, o.opt.jacobi_scaling);
+  LmStep st;
+  if (!lm_step(ne, s, radius, o.opt, false, st)) { o.err = "Cholesky breakdown"; return ICC_ERR_NUMERIC; }
+  if (cost) *cost = c;
+  for (int i = 0; i < n; ++i) {
+    const int j = o.perm[i];
+    if (gradient) gradient[i] = ne.g[j];
+    if (scale) scale[i] = s[j];
+    if (lm_diag) lm_diag[i] = st.D2[j];
+    if (delta) delta[i] = st.y[j] * s[j];
+  }
+  if (hessian_dense) for (int i = 0; i < n; ++i) for (int j = 0; j < n; ++j) hessian_dense[size_t(i) * n + j] = ne.get(o.perm[i], o.perm[j]);
+  if (model_change) *model_change = st.model_change;
   return ICC_OK;
 }
 
