@@ -351,6 +351,30 @@ icc_status icc_calibrate_camera(icc_handle* h, int model, int image_width, int i
                                 double focal_length_init, double distortion_init, const icc_camcal_options* options /* nullable */,
                                 double* intrinsics /* 10 */, double* q_wc_xyzw, double* p_wc, double* view_reproj_error_px, int32_t* view_used,
                                 icc_camcal_summary* summary /* nullable */);
+/* One iteration body of icc_calibrate_camera's bundle adjustment at a given state (test surface): the normal equations, the damped
+ * step at `radius`, the cost at the candidate, and the per-view mean reprojection error at the current state, through the same
+ * launches the calibration runs.  Nothing of the handle changes except its last error.
+ * Inputs: views in CSR form over the handle's board points; per view q_wc (x,y,z,w; normalised here) and p_wc as
+ * icc_calibrate_camera takes them; intrinsics[10] in Theia order; `active`: n_active distinct view indices in any order (slot s
+ * holds view active[s]); intr_mask: free intrinsics (bit i = Theia parameter i); pose_free; huber_width; scale_in: the Jacobi
+ * scale (6 n_active + 10) of an earlier iteration of the stage, or NULL to compute it as on a stage's first iteration.
+ * Tangent of slot s: [delta (right increment of R_cw = conj(q_wc)) | camera centre], then the free intrinsics in Theia order.
+ * Outputs, each nullable: blocks (n_active x 153, slot-major): packed upper triangle (row by row) of slot s's 17 x 17
+ * [J_pose | J_intr | r]^T [J_pose | J_intr | r] with Huber-weighted rows; sys (154): the sum over slots of the intrinsics part
+ * (rows 6..16 of the same packing, other entries 0) and the cost; red (66): the Schur complement of the poses onto the intrinsics,
+ * packed upper 10 x 10 (55) then the gradient part (10); Y (n_active x 66): A_s^-1 [H_pk | g_p] (6 x 11, row-major), A_s the
+ * damped pose block; scale (6 n_active + 10): the scale used; dk (10): intrinsics step; scalars (8): candidate cost, g.delta,
+ * delta^T D delta, |delta|^2, x^2, failed factorisations, max |g|, cost; q_wc_cand / p_wc_cand (n_views) and intr_cand (10): the
+ * candidate state (inactive views unchanged); view_error_px (n_views): mean reprojection error of the active views at the current
+ * state, 0 elsewhere. */
+typedef struct icc_camcal_step_out {
+  double* blocks; double* sys; double* red; double* Y; double* scale; double* dk; double* scalars;
+  double* q_wc_cand; double* p_wc_cand; double* intr_cand; double* view_error_px;
+} icc_camcal_step_out;
+icc_status icc_camcal_step(icc_handle* h, int model, int n_views, const int32_t* corner_offsets, const int32_t* point_ids, const double* uv,
+                           const double* q_wc_xyzw, const double* p_wc, const double* intrinsics, int n_active, const int32_t* active,
+                           uint32_t intr_mask, int pose_free, double huber_width, double radius, const double* scale_in /* nullable */,
+                           icc_camcal_step_out* out);
 
 /* ---- upstream: static IMU biases, the `--imu_bias_file` input of the hot CLI ------------------------------------------------------------
  * python/get_imu_biases.py:36-53: gyroscope bias = mean of the gyroscope stream; accelerometer bias = mean of the accelerometer stream

@@ -73,7 +73,16 @@ class CamCalSummary(C.Structure):
         return d
 
 
-ALLREDUCE_FN = C.CFUNCTYPE(None, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p)
+class CamCalStepOut(C.Structure):
+    """icc_camcal_step_out (include/icc_b200.h): caller-owned output arrays, each nullable."""
+    _fields_ = [(k, c_double_p) for k in ("blocks", "sys", "red", "Y", "scale", "dk", "scalars", "q_wc_cand", "p_wc_cand", "intr_cand", "view_error_px")]
+
+
+CC_PACK, CC_Y = 153, 66    # packed upper triangle of a view's 17 x 17 [J | r] block; A^-1 [H_pk | g_p] (6 x 11)
+CAMCAL_SCALARS = ("cand_cost", "g_delta", "d_delta", "step_sq", "x_sq", "fail", "grad_max", "x_cost")
+
+
+ALLREDUCE_FN =C.CFUNCTYPE(None, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p)
 
 
 class IccError(RuntimeError):
@@ -221,6 +230,29 @@ class CApi:
                    float(focal_length_init), float(distortion_init), C.byref(o), _dp(intr), _dp(q), _dp(p), _dp(e), used.ctypes.data_as(c_int32_p), C.byref(s))
         from .camera_models import NUM_PARAMS
         return dict(intrinsics=intr[:NUM_PARAMS[int(model)]], q_wc=q, p_wc=p, view_error_px=e, used=used, summary=s.as_dict())
+
+    def camcal_step(self, model, corner_offsets, point_ids, uv, q_wc, p_wc, intrinsics, active, intr_mask, pose_free, radius,
+                    huber_width=1.345, scale_in=None):
+        """One iteration body of the camera calibration's bundle adjustment at a given state (icc_camcal_step) -> dict of blocks
+        (n_active, 153), sys (154), red (66), Y (n_active, 6, 11), scale (6 n_active + 10), dk (10), scalars (CAMCAL_SCALARS),
+        q_wc_cand, p_wc_cand, intr_cand (10), view_error_px; board points must be set."""
+        off = np.ascontiguousarray(corner_offsets, dtype=np.int32); ids = np.ascontiguousarray(point_ids, dtype=np.int32); uv = _f64(uv)
+        act = np.ascontiguousarray(active, dtype=np.int32)
+        nv, na = off.size - 1, act.size
+        q, p, k = _f64(q_wc).reshape(nv, 4), _f64(p_wc).reshape(nv, 3), _f64(intrinsics)
+        assert ids.size == off[-1] and uv.size == 2 * ids.size and k.size == 10
+        si = None if scale_in is None else _f64(scale_in)
+        assert si is None or si.size == 6 * na + 10
+        r = dict(blocks=np.zeros((na, CC_PACK)), sys=np.zeros(CC_PACK + 1), red=np.zeros(66), Y=np.zeros((na, 6, 11)), scale=np.zeros(6 * na + 10),
+                 dk=np.zeros(10), scalars=np.zeros(len(CAMCAL_SCALARS)), q_wc_cand=np.zeros((nv, 4)), p_wc_cand=np.zeros((nv, 3)),
+                 intr_cand=np.zeros(10), view_error_px=np.zeros(nv))
+        out = CamCalStepOut(*(_dp(r[f]) for f, _ in CamCalStepOut._fields_))
+        self._call("camcal_step", [C.c_int, C.c_int, c_int32_p, c_int32_p, c_double_p, c_double_p, c_double_p, c_double_p, C.c_int, c_int32_p,
+                                   C.c_uint32, C.c_int, C.c_double, C.c_double, c_double_p, C.POINTER(CamCalStepOut)],
+                   int(model), nv, off.ctypes.data_as(c_int32_p), ids.ctypes.data_as(c_int32_p), _dp(uv), _dp(q), _dp(p), _dp(k), na,
+                   act.ctypes.data_as(c_int32_p), int(intr_mask), int(pose_free), float(huber_width), float(radius), _dp(si), C.byref(out))
+        r["scalars"] = dict(zip(CAMCAL_SCALARS, r["scalars"]))
+        return r
 
     # ---- upstream row f3: ImuToCameraRotationEstimator (src/core/imu_to_camera_rotation_estimator.cc:116-274) -----------------
     def estimate_imu_to_camera_rotation(self, view_t_s, q_cw_xyzw, imu_t_s, gyro, gyro_bias=None):

@@ -1828,6 +1828,41 @@ IntrinsicSubsets intrinsic_subsets(int model) {
     default: return {0u, 0u, 0u, 0u, 0u};
   }
 }
+
+// board points (the handle's), corner offsets, point ids and pixels of a camera calibration, on the device
+struct CamCalInputs { DevBuf<double4> board; DevBuf<int> off, pid; DevBuf<double2> uv; };
+icc_status upload_camcal_inputs(icc_handle* h, int nv, const int32_t* off, const int32_t* ids, const double* uv, CamCalInputs& in) {
+  const int nc = off[nv], np = (int)(h->points.size() / 4);
+  cudaStream_t st = h->stream;
+  std::vector<double4> board(np);
+  for (int i = 0; i < np; ++i) board[i] = make_double4(h->points[4 * i], h->points[4 * i + 1], h->points[4 * i + 2], h->points[4 * i + 3]);
+  CU(in.board.upload(board));
+  CU(in.off.alloc(nv + 1)); CU(in.pid.alloc(std::max(1, nc))); CU(in.uv.alloc(std::max(1, nc)));
+  CU(cudaMemcpyAsync(in.off.p, off, (size_t)(nv + 1) * sizeof(int), cudaMemcpyHostToDevice, st));
+  if (nc > 0) {
+    CU(cudaMemcpyAsync(in.pid.p, ids, (size_t)nc * sizeof(int), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(in.uv.p, uv, (size_t)nc * sizeof(double2), cudaMemcpyHostToDevice, st));
+  }
+  return ICC_OK;
+}
+
+// device buffers of one bundle-adjustment iteration (sizes as in launch_camcal_accumulate / launch_camcal_step)
+struct CamCalStepBufs { double *blocks, *sys, *red, *Y, *scale, *dk, *scal; };
+// One iteration body of bundle_adjust: with `evaluate` the normal equations at `cur` (per-slot blocks, sys with the cost), then the
+// damped step at `radius` into `cand` with its scalars, and the cost at `cand` into scal[CC_CAND_COST].
+cudaError_t launch_camcal_iteration(const CamCalProblem& Q, const CamCalState& cur, const CamCalState& cand, const CamCalStepBufs& b,
+                                    bool evaluate, bool compute_scale, double radius, cudaStream_t st) {
+  cudaError_t e;
+  if (evaluate) {
+    if ((e = cudaMemsetAsync(b.sys, 0, (CC_PACK + 1) * sizeof(double), st)) != cudaSuccess) return e;
+    launch_camcal_accumulate(Q, cur, true, b.blocks, b.sys, nullptr, nullptr, st);
+  }
+  if ((e = cudaMemsetAsync(b.red, 0, 66 * sizeof(double), st)) != cudaSuccess) return e;
+  if ((e = cudaMemsetAsync(b.scal, 0, CC_SCAL_COUNT * sizeof(double), st)) != cudaSuccess) return e;
+  launch_camcal_step(Q, cur, cand, b.blocks, b.sys, b.red, b.Y, b.scale, compute_scale ? 1 : 0, radius, 1e-6, 1e32, b.dk, b.scal, st);
+  launch_camcal_accumulate(Q, cand, false, nullptr, nullptr, b.scal + CC_CAND_COST, nullptr, st);
+  return cudaSuccess;
+}
 }  // namespace
 
 icc_status icc_calibrate_camera(icc_handle* h, int model, int W, int H, int nv, const int32_t* off, const int32_t* ids, const double* uv,
@@ -1859,16 +1894,11 @@ icc_status icc_calibrate_camera(icc_handle* h, int model, int W, int H, int nv, 
   CU(cudaSetDevice(h->device));
   cudaStream_t st = h->stream;
   // ---- inputs to the device ------------------------------------------------------------------------------------------------
-  std::vector<double4> board(np);
-  for (int i = 0; i < np; ++i) board[i] = make_double4(h->points[4 * i], h->points[4 * i + 1], h->points[4 * i + 2], h->points[4 * i + 3]);
-  DevBuf<double4> d_board; DevBuf<int> d_off, d_pid, d_active; DevBuf<double2> d_uv;
-  CU(d_board.upload(board));
-  CU(d_off.alloc(nv + 1)); CU(d_pid.alloc(std::max(1, nc))); CU(d_uv.alloc(std::max(1, nc))); CU(d_active.alloc(nv));
-  CU(cudaMemcpyAsync(d_off.p, off, (size_t)(nv + 1) * sizeof(int), cudaMemcpyHostToDevice, st));
-  if (nc > 0) {
-    CU(cudaMemcpyAsync(d_pid.p, ids, (size_t)nc * sizeof(int), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(d_uv.p, uv, (size_t)nc * sizeof(double2), cudaMemcpyHostToDevice, st));
-  }
+  CamCalInputs in;
+  { const icc_status r = upload_camcal_inputs(h, nv, off, ids, uv, in); if (r != ICC_OK) return r; }
+  DevBuf<double4>& d_board = in.board; DevBuf<int>& d_off = in.off; DevBuf<int>& d_pid = in.pid; DevBuf<double2>& d_uv = in.uv;
+  DevBuf<int> d_active;
+  CU(d_active.alloc(nv));
   const double cx0 = W / 2.0, cy0 = H / 2.0;                       // AddView (:99)
   // ---- initial focal length and poses ----------------------------------------------------------------------------------------
   std::vector<double> q0(4 * (size_t)nv), p0(3 * (size_t)nv); std::vector<int> ok0(nv, 1);
@@ -1921,6 +1951,7 @@ icc_status icc_calibrate_camera(icc_handle* h, int model, int W, int H, int nv, 
   const size_t na0 = std::max<size_t>(1, active.size());
   CU(d_blocks.alloc(na0 * CC_PACK)); CU(d_Y.alloc(na0 * CC_Y)); CU(d_scale.alloc(6 * na0 + 10)); CU(d_sys.alloc(CC_PACK + 1)); CU(d_red.alloc(66));
   CU(d_dk.alloc(10)); CU(d_scal.alloc(CC_SCAL_COUNT)); CU(d_verr.alloc(nv));
+  const CamCalStepBufs bufs{d_blocks.p, d_sys.p, d_red.p, d_Y.p, d_scale.p, d_dk.p, d_scal.p};
   int cur = 0;
   CamCalProblem Q; memset(&Q, 0, sizeof Q);
   Q.model = model; Q.n_points = np; Q.huber = o.huber_width; Q.board = d_board.p; Q.f_off = d_off.p; Q.pid = d_pid.p; Q.uv = d_uv.p; Q.active = d_active.p;
@@ -1955,16 +1986,9 @@ icc_status icc_calibrate_camera(icc_handle* h, int model, int W, int H, int nv, 
     int term = 0, iters = 0;
     if (Q.n_active == 0 || (mask == 0u && !pose_free)) { if (stage >= 0) S.termination[stage] = 3; return ICC_OK; }
     for (int it = 0; it < o.max_num_iterations; ++it) {
-      bool fresh = false;
-      if (!ne_valid) {
-        CU(cudaMemsetAsync(d_sys.p, 0, (CC_PACK + 1) * sizeof(double), st));
-        launch_camcal_accumulate(Q, state(cur), true, d_blocks.p, d_sys.p, nullptr, nullptr, st);
-        ne_valid = true; fresh = true;
-      }
-      CU(cudaMemsetAsync(d_red.p, 0, 66 * sizeof(double), st));
-      CU(cudaMemsetAsync(d_scal.p, 0, CC_SCAL_COUNT * sizeof(double), st));
-      launch_camcal_step(Q, state(cur), state(1 - cur), d_blocks.p, d_sys.p, d_red.p, d_Y.p, d_scale.p, first ? 1 : 0, radius, 1e-6, 1e32, d_dk.p, d_scal.p, st);
-      launch_camcal_accumulate(Q, state(1 - cur), false, nullptr, nullptr, d_scal.p + CC_CAND_COST, nullptr, st);
+      const bool fresh = !ne_valid;
+      CU(launch_camcal_iteration(Q, state(cur), state(1 - cur), bufs, fresh, first, radius, st));
+      ne_valid = true;
       CU(cudaMemcpyAsync(sc, d_scal.p, sizeof sc, cudaMemcpyDeviceToHost, st));
       CU(cudaStreamSynchronize(st));
       if (fresh) {
@@ -2106,7 +2130,7 @@ icc_status icc_calibrate_camera(icc_handle* h, int model, int W, int H, int nv, 
     PQ.normalized = 0; PQ.n_points = np; PQ.min_obs = 1; PQ.huber = o.huber_width;
     PQ.board_in = d_board.p; PQ.pt_off = d_pt_off.p; PQ.pt_obs = d_pt_obs.p; PQ.obs_view = d_view.p; PQ.meas = d_uv.p; PQ.q_cw = d_q[cur].p; PQ.cam_c = d_c[cur].p;
     launch_point_refine(PQ, d_board2.p, d_opt.p, st);
-    std::vector<int> opt(np);
+    std::vector<int> opt(np); std::vector<double4> board(np);
     CU(cudaMemcpyAsync(d_board.p, d_board2.p, (size_t)np * sizeof(double4), cudaMemcpyDeviceToDevice, st));
     CU(cudaMemcpyAsync(board.data(), d_board2.p, (size_t)np * sizeof(double4), cudaMemcpyDeviceToHost, st));
     CU(cudaMemcpyAsync(opt.data(), d_opt.p, (size_t)np * sizeof(int), cudaMemcpyDeviceToHost, st));
@@ -2118,6 +2142,60 @@ icc_status icc_calibrate_camera(icc_handle* h, int model, int W, int H, int nv, 
     S.iterations[2] += it3;
   }
   return finish(true);
+}
+
+icc_status icc_camcal_step(icc_handle* h, int model, int nv, const int32_t* off, const int32_t* ids, const double* uv,
+                           const double* q_wc, const double* p_wc, const double* intrinsics, int n_active, const int32_t* active,
+                           uint32_t intr_mask, int pose_free, double huber_width, double radius, const double* scale_in,
+                           icc_camcal_step_out* out) {
+  if (!h || nv <= 0 || !off || !ids || !uv || !q_wc || !p_wc || !intrinsics || n_active <= 0 || !active || !out) return ICC_ERR_INVALID_ARGUMENT;
+  if (intr_mask >= (1u << 10) || !(huber_width > 0.0) || !(radius > 0.0)) return ICC_ERR_INVALID_ARGUMENT;
+  NEED_DEVICE();
+  if (camera_num_params(model) < 0) return fail(h, ICC_ERR_INVALID_ARGUMENT, "unknown camera model");
+  if (h->points.empty()) return fail(h, ICC_ERR_STATE, "icc_set_board_points must be called first");
+  if (off[0] != 0) return fail(h, ICC_ERR_INVALID_ARGUMENT, "corner offsets must start at 0");
+  for (int i = 0; i < nv; ++i) if (off[i + 1] < off[i]) return fail(h, ICC_ERR_INVALID_ARGUMENT, "corner offsets must be non-decreasing");
+  const int nc = off[nv], np = (int)(h->points.size() / 4);
+  for (int i = 0; i < nc; ++i) if (ids[i] < 0 || ids[i] >= np) return fail(h, ICC_ERR_INVALID_ARGUMENT, "point id outside the board");
+  std::vector<char> seen(nv, 0);
+  for (int s = 0; s < n_active; ++s) {
+    if (active[s] < 0 || active[s] >= nv || seen[active[s]]) return fail(h, ICC_ERR_INVALID_ARGUMENT, "active views must be distinct view indices");
+    seen[active[s]] = 1;
+  }
+  CU(cudaSetDevice(h->device));
+  cudaStream_t st = h->stream;
+  CamCalInputs in;
+  { const icc_status r = upload_camcal_inputs(h, nv, off, ids, uv, in); if (r != ICC_OK) return r; }
+  std::vector<double> qs(4 * (size_t)nv), cs(p_wc, p_wc + 3 * (size_t)nv), ks(intrinsics, intrinsics + 10);
+  for (int v = 0; v < nv; ++v) { const Q4 q = qn(&q_wc[4 * v]); qs[4 * v] = -q.x; qs[4 * v + 1] = -q.y; qs[4 * v + 2] = -q.z; qs[4 * v + 3] = q.w; }
+  const size_t na = (size_t)n_active;
+  DevBuf<int> d_active; DevBuf<double> d_q[2], d_c[2], d_k[2], d_blocks, d_Y, d_scale, d_sys, d_red, d_dk, d_scal, d_verr, d_vcost;
+  CU(d_active.upload(std::vector<int>(active, active + n_active)));
+  for (int i = 0; i < 2; ++i) { CU(d_q[i].upload(qs)); CU(d_c[i].upload(cs)); CU(d_k[i].upload(ks)); }
+  CU(d_blocks.alloc(na * CC_PACK)); CU(d_Y.alloc(na * CC_Y)); CU(d_scale.alloc(6 * na + 10)); CU(d_sys.alloc(CC_PACK + 1)); CU(d_red.alloc(66));
+  CU(d_dk.alloc(10)); CU(d_scal.alloc(CC_SCAL_COUNT)); CU(d_verr.alloc(nv)); CU(d_vcost.alloc(1));
+  if (scale_in) CU(cudaMemcpyAsync(d_scale.p, scale_in, (6 * na + 10) * sizeof(double), cudaMemcpyHostToDevice, st));
+  else CU(cudaMemsetAsync(d_scale.p, 0, (6 * na + 10) * sizeof(double), st));   // poses constant: the view part stays 0
+  CamCalProblem Q; memset(&Q, 0, sizeof Q);
+  Q.model = model; Q.n_points = np; Q.n_active = n_active; Q.pose_free = pose_free ? 1 : 0; Q.intr_mask = intr_mask; Q.huber = huber_width;
+  Q.board = in.board.p; Q.f_off = in.off.p; Q.pid = in.pid.p; Q.uv = in.uv.p; Q.active = d_active.p;
+  const CamCalState cur{d_q[0].p, d_c[0].p, d_k[0].p}, cand{d_q[1].p, d_c[1].p, d_k[1].p};
+  const CamCalStepBufs bufs{d_blocks.p, d_sys.p, d_red.p, d_Y.p, d_scale.p, d_dk.p, d_scal.p};
+  CU(launch_camcal_iteration(Q, cur, cand, bufs, true, scale_in == nullptr, radius, st));
+  // GetReprojErrorOfView at the current state, as view_errors() of icc_calibrate_camera reads it
+  CU(cudaMemsetAsync(d_verr.p, 0, (size_t)nv * sizeof(double), st)); CU(cudaMemsetAsync(d_vcost.p, 0, sizeof(double), st));
+  launch_camcal_accumulate(Q, cur, false, nullptr, nullptr, d_vcost.p, d_verr.p, st);
+  CU(cudaGetLastError());
+  auto get = [&](double* dst, const double* src, size_t n) { return dst ? cudaMemcpyAsync(dst, src, n * sizeof(double), cudaMemcpyDeviceToHost, st) : cudaSuccess; };
+  CU(get(out->blocks, d_blocks.p, na * CC_PACK)); CU(get(out->sys, d_sys.p, CC_PACK + 1)); CU(get(out->red, d_red.p, 66)); CU(get(out->Y, d_Y.p, na * CC_Y));
+  CU(get(out->scale, d_scale.p, 6 * na + 10)); CU(get(out->dk, d_dk.p, 10)); CU(get(out->scalars, d_scal.p, CC_SCAL_COUNT));
+  CU(get(out->intr_cand, d_k[1].p, 10)); CU(get(out->p_wc_cand, d_c[1].p, 3 * (size_t)nv)); CU(get(out->view_error_px, d_verr.p, nv));
+  std::vector<double> qc(4 * (size_t)nv);
+  CU(get(out->q_wc_cand ? qc.data() : nullptr, d_q[1].p, qc.size()));
+  CU(cudaStreamSynchronize(st));
+  if (out->q_wc_cand)
+    for (int v = 0; v < nv; ++v) { out->q_wc_cand[4 * v] = -qc[4 * v]; out->q_wc_cand[4 * v + 1] = -qc[4 * v + 1]; out->q_wc_cand[4 * v + 2] = -qc[4 * v + 2]; out->q_wc_cand[4 * v + 3] = qc[4 * v + 3]; }
+  return ICC_OK;
 }
 
 // ---- upstream: static IMU biases (python/get_imu_biases.py:36-53) -------------------------------------------------------------------

@@ -2213,4 +2213,31 @@ icc_status icco_estimate_imu_biases(void* h, int n, const double* acc, const dou
 
 int icco_project(int model, const double* intr, const double* p3, double* px, int dispatch_fov) { return project<double>(model, intr, p3, px, dispatch_fov != 0) ? 1 : 0; }
 
+// n camera-frame points through project<T> (FOV dispatched, as the CUDA calibration does) with Jet<4> passes over the 13 inputs
+// [point (3) | intrinsics (10)]: pixel px[2n], point Jacobian Jp[6n] (2 x 3 row-major per point), intrinsic Jacobian Jk[20n]
+// (2 x 10 row-major), ok[n].  Returns the number of points that project.
+int icco_project_jacobian(int model, const double* intr, int n, const double* p3, double* px, double* Jp, double* Jk, int32_t* ok) {
+  typedef Jet<4> J4;
+  int n_ok = 0;
+  for (int i = 0; i < n; ++i) {
+    bool good = true;
+    for (int pass = 0; pass < 4; ++pass) {
+      J4 p[3], k[10], r[2];
+      for (int a = 0; a < 3; ++a) { p[a] = J4(p3[3 * i + a]); if (a / 4 == pass) p[a].v[a % 4] = 1.0; }
+      for (int a = 0; a < 10; ++a) { k[a] = J4(intr[a]); if ((3 + a) / 4 == pass) k[a].v[(3 + a) % 4] = 1.0; }
+      good = project<J4>(model, k, p, r, true) && good;
+      for (int row = 0; row < 2; ++row) {
+        px[2 * i + row] = r[row].a;
+        for (int d = 0; d < 4; ++d) {
+          const int col = 4 * pass + d;
+          if (col < 3) Jp[6 * i + 3 * row + col] = r[row].v[d];
+          else if (col < 13) Jk[20 * i + 10 * row + col - 3] = r[row].v[d];
+        }
+      }
+    }
+    ok[i] = good ? 1 : 0; n_ok += good;
+  }
+  return n_ok;
+}
+
 }  // extern "C"

@@ -40,6 +40,7 @@ def test_no_cpu_fallback_without_device():
     for call in (lambda: h.optimize(1, 66), lambda: h.evaluate(66), lambda: h.lm_iterations(1, 66), lambda: h.mean_reprojection_error(),
                  lambda: h.eval_trajectory([0]), lambda: h.time_evaluations(1, 66),
                  lambda: h.calibrate_camera(0, 960, 540, [0, 1], [0], [[1.0, 2.0]]), lambda: h.estimate_imu_biases(np.ones((4, 3)), np.ones((4, 3))),
+                 lambda: h.camcal_step(0, [0, 1], [0], [[1.0, 2.0]], [[0, 0, 0, 1.0]], [[0, 0, 1.0]], np.ones(10), [0], 1, 1, 1e4),
                  lambda: h.optimize_board_points([0, 1], [0], [[1.0, 2.0]], [[0, 0, 0, 1.0]], [[0, 0, 1.0]], [1])):
         with pytest.raises(capi.IccError, match="ICC_ERR_NO_DEVICE"):
             call()

@@ -57,14 +57,18 @@ def load(api, name):
     return api
 
 
-def damped_solve_reference(H, g, radius, jacobi=True, min_diag=1e-6, max_diag=1e32, refinements=3):
+def damped_solve_reference(H, g, radius, jacobi=True, min_diag=1e-6, max_diag=1e32, refinements=3, scale=None):
     """NumPy statement of one Levenberg-Marquardt step of Ceres (Jacobi scaling + clamped diagonal), solved densely in high precision:
-    S = diag(1 / (1 + sqrt(H_ii))) (identity without Jacobi scaling), D = diag(clamp(diag(S H S), min, max) / radius),
+    S = diag(1 / (1 + sqrt(H_ii))) (identity without Jacobi scaling; `scale` when given, e.g. the scale of a stage's first
+    iteration reused on a later one), D = diag(clamp(diag(S H S), min, max) / radius),
     A = S H S + D, b = -S g; y from a float64 Cholesky plus `refinements` rounds of iterative refinement with the residual
     accumulated in long double.  -> dict(scale, lm_diag, A, b, y, delta = S y, model_change = 1/2 (y^T D y - y^T S g))."""
     from scipy.linalg import cho_factor, cho_solve
     H = np.asarray(H, dtype=np.float64); g = np.asarray(g, dtype=np.float64)
-    s = 1.0 / (1.0 + np.sqrt(np.diag(H))) if jacobi else np.ones(len(g))
+    if scale is not None:
+        s = np.asarray(scale, dtype=np.float64)
+    else:
+        s = 1.0 / (1.0 + np.sqrt(np.diag(H))) if jacobi else np.ones(len(g))
     SHS = H * s[:, None] * s[None, :]
     D = np.minimum(np.maximum(np.diag(SHS), min_diag), max_diag) / radius
     A = SHS + np.diag(D)
